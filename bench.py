@@ -55,6 +55,27 @@ SAMPLES_PER_FRAME = OUT_HW[0] * OUT_HW[1] * SPP
 PIX_PER_FRAME = OUT_HW[0] * OUT_HW[1]
 
 
+DUMP_CAP_BYTES = 64 * 10**6
+
+
+def write_dump(dirname, arrays):
+    """--dump-outputs: every array as DIR/<name>.npy in float32.  Over DUMP_CAP_BYTES in all, each array is replaced by the
+    same seeded sample of its flattened elements on every run (DIR/<name>.npy) and their flat indices (DIR/<name>_index.npy,
+    float64), the two together kept within the cap."""
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(a.size * 4 for a in arrays.values())
+    budget = DUMP_CAP_BYTES - 2 * 4096 * len(arrays)                     # room for the .npy headers
+    for seed, (name, a) in enumerate(sorted(arrays.items())):
+        flat = np.ascontiguousarray(a, dtype=np.float32).reshape(-1)
+        if total <= budget:
+            np.save(os.path.join(dirname, name + '.npy'), flat.reshape(a.shape))
+            continue
+        n = int(flat.size * budget // (3 * total))                        # 4 B of value + 8 B of index per kept element
+        idx = np.sort(np.random.default_rng(seed).choice(flat.size, size=n, replace=False))
+        np.save(os.path.join(dirname, name + '.npy'), flat[idx])
+        np.save(os.path.join(dirname, name + '_index.npy'), idx.astype(np.float64))
+
+
 def measured_peaks():
     p = os.path.join(ROOT, 'MEASURED_PEAKS.json')
     if os.path.exists(p):
@@ -379,6 +400,11 @@ def run_gpu_arm(args):
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_begin
     launches = int(L.sdb_launch_count()) - launches0
+    if args.dump_outputs and rank == 0:                              # the host result of the last timed step, before anything reuses it
+        if e2e_image:
+            dump = {'rgb': host_rgb.numpy().copy()}
+        else:
+            dump = {'depth': host_out[0, :res[0]].numpy().copy(), 'opacity': host_out[1, :res[0]].numpy().copy()}
     if world_size > 1:
         dist.barrier()
     step_ms = [a.elapsed_time(b) for a, b in evs]
@@ -517,6 +543,8 @@ def run_gpu_arm(args):
                            'ms_per_step_incl_wait_for_slowest_rank': float(np.mean(coll_ms))} if world_size > 1 else None,
         }
         line.update(extras)
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, dump)
         print(json.dumps(line))
     if world_size > 1:
         dist.destroy_process_group()
@@ -589,7 +617,14 @@ def main():
     ap.add_argument('--no-extras', action='store_true', help='skip the C4 / C5 / reference-CUDA legs reported next to the headline at N=1')
     ap.add_argument('--no-early-stop', action='store_true',
                     help='march every sample of every live tile (early termination off; the reference arithmetic sample for sample)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the host result of the last timed step (rank 0: in weak mode with several GPUs, its own frame) to '
+                         'DIR/<name>.npy in float32: rgb [3,H,W], or in strong mode depth and opacity [rows,W].  Over 64 MB in all, '
+                         'a fixed seeded sample of the flattened elements is written instead, with its flat indices in '
+                         'DIR/<name>_index.npy (float64).  The inputs depend on the arguments alone')
     args = ap.parse_args()
+    if args.impl == 'reference' and args.dump_outputs:
+        ap.error('--dump-outputs writes what the CUDA path computed; the reference arm has nothing to dump')
     if args.impl == 'reference':
         run_reference_arm(args)
         return

@@ -23,4 +23,5 @@ def golden_ops():
 @pytest.fixture(scope='session')
 def golden_fpp():
     import numpy as np
-    return np.load(os.path.join(GOLDEN, 'ref_forward_perpix.npz'))
+    # two files, each under 1 MB: the frame inputs + the 'spec' parameter set, and the 'stress' set
+    return {**np.load(os.path.join(GOLDEN, 'ref_forward_perpix.npz')), **np.load(os.path.join(GOLDEN, 'ref_forward_perpix_stress.npz'))}

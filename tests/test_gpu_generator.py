@@ -193,33 +193,56 @@ def test_fused_camera_sampler_reproduces_the_reference(fused_generator):
         del gen.voxel.sample_world
 
 
-def test_world_builder_reproduces_next_world(fused_generator, tmp_path):
-    """f3: PCGVoxelGenerator.next_world through the hook (volume built in HBM) == the reference's own CPU next_world on the same
-    bird's-eye-view files and tree assets: voxel volume, height map, world offset and both conditioning maps, bit for bit."""
-    import random
+WORLD_SIZE = 320
+
+
+def world_builder_inputs(d):
+    """Bird's-eye-view files of a WORLD_SIZE^2 scene written to directory `d`, and the tree assets."""
     import cv2
-    import imaginaire.model_utils.pcg_gen as pcg
     from scenedreamer_b200 import synth
-    assert '_sdb200_reference_next_world' in pcg.PCGVoxelGenerator.__dict__          # armed together with the generator hook
-    size = 320
-    h, sem, tree = synth.make_bev(size, seed=11)
+    h, sem, tree = synth.make_bev(WORLD_SIZE, seed=11)
     tree[::5, ::7] = np.where(sem[::5, ::7] != 9, sem[::5, ::7], 255)               # denser trees: overlapping models
-    d = str(tmp_path)
     np.save(os.path.join(d, 'heightmap.npy'), h)
     cv2.imwrite(os.path.join(d, 'semanticmap.png'), sem)
     cv2.imwrite(os.path.join(d, 'treemap.png'), tree)
-    assets = {'assets': [torch.from_numpy(m) for m in synth.make_tree_models()]}
-    ref, ours = pcg.PCGVoxelGenerator(size), pcg.PCGVoxelGenerator(size)
+    return {'assets': [torch.from_numpy(m) for m in synth.make_tree_models()]}
+
+
+def test_world_builder_reproduces_next_world(tmp_path, request):
+    """f3: PCGVoxelGenerator.next_world through the hook (volume built in HBM) == the reference's own CPU next_world on the same
+    bird's-eye-view files and tree assets (stored by tests/golden/make_golden_world.py): voxel volume, height map, world offset
+    and both conditioning maps, bit for bit, and the host RNG left where the reference leaves it."""
+    import random
+    import types
+    import _golden
+    from scenedreamer_b200 import worldgen
+    d = str(tmp_path)
+    assets = world_builder_inputs(d)
+    g = np.load(os.path.join(ROOT, 'tests', 'golden', 'ref_world.npz'))
+    ours = types.SimpleNamespace()
     random.seed(7)
-    pcg.PCGVoxelGenerator._sdb200_reference_next_world(ref, 'cpu', d, assets)
-    state_after_ref = random.getstate()
-    random.seed(7)
-    ours.next_world(torch.device(DEV), d, assets)
-    assert random.getstate() == state_after_ref                                     # random.choice consumed identically
+    worldgen.fused_next_world(ours, torch.device(DEV), d, assets)
+    assert list(random.getstate()[1]) == g['rng_state'].tolist()                      # random.choice consumed identically
     assert ours.voxel_t.is_cuda and ours.voxel_t.dtype == torch.int32
-    assert torch.equal(ours.voxel_t.cpu(), ref.voxel_t)
-    assert torch.equal(ours.heightmap, ref.heightmap) and ours.heightmap.dtype == ref.heightmap.dtype
-    assert torch.equal(ours.trans_mat, ref.trans_mat)
-    assert torch.equal(ours.current_height_map.cpu(), ref.current_height_map)
-    assert torch.equal(ours.current_semantic_map.cpu(), ref.current_semantic_map)
+    assert list(ours.voxel_t.shape) == g['voxel_t_shape'].tolist()
+    _golden.check_exact(g, 'voxel_t', ours.voxel_t)
+    _golden.check_exact(g, 'heightmap', ours.heightmap)
+    assert torch.equal(ours.trans_mat, torch.from_numpy(g['trans_mat']))
+    _golden.check_exact(g, 'current_height_map', ours.current_height_map)
+    _golden.check_exact(g, 'current_semantic_map', ours.current_semantic_map)
     assert int((ours.voxel_t == 17).sum()) > 0 and int((ours.voxel_t == 18).sum()) > 0   # trees really got pasted
+    if _have_reference():                                                             # armed together with the generator hook
+        request.getfixturevalue('fused_generator')
+        import imaginaire.model_utils.pcg_gen as pcg
+        assert '_sdb200_reference_next_world' in pcg.PCGVoxelGenerator.__dict__
+        assert pcg.PCGVoxelGenerator.next_world is worldgen.fused_next_world
+        routed = pcg.PCGVoxelGenerator(WORLD_SIZE)                                    # the reference's own entry point
+        random.seed(7)
+        routed.next_world(torch.device(DEV), d, assets)
+        assert list(random.getstate()[1]) == g['rng_state'].tolist()
+        assert routed.voxel_t.is_cuda
+        _golden.check_exact(g, 'voxel_t', routed.voxel_t)
+        _golden.check_exact(g, 'heightmap', routed.heightmap)
+        assert torch.equal(routed.trans_mat, torch.from_numpy(g['trans_mat']))
+        _golden.check_exact(g, 'current_height_map', routed.current_height_map)
+        _golden.check_exact(g, 'current_semantic_map', routed.current_semantic_map)
